@@ -2,9 +2,12 @@
 """bench.py -- R-GCN layer fwd+bwd throughput (M-edges/s) on B200, one process per GPU.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--scale S] [--impl ours|reference]
+                  [--dump-outputs DIR]
 
 A "step" is ONE pass of the hot path over one graph: one block-diagonal R-GCN layer forward + backward
-(dH, dW_forward, dW_backward, dW_self) on synthetic data of the named shape.
+(dH, dW_forward, dW_backward, dW_self) on synthetic data of the named shape.  K timed steps follow W warm-up steps.
+--dump-outputs DIR writes what the last timed step returned (out, dH, dW_forward, dW_backward, dW_self) as
+DIR/<name>.npy, so that two builds can be compared output for output on the same seeded inputs (see dump_outputs).
 Metric (BASELINE.json): M-edges/s = triples E / (t_fwd + t_bwd) / 1e6, graph prep excluded from `value`
 (device-resident inputs) and INCLUDED in `e2e` (host buffers in, host buffers out).
 
@@ -274,6 +277,25 @@ def relerr(a, b):
     return float((a - b).abs().max() / (b.abs().max() + 1e-30))
 
 
+DUMP_BYTES_PER_ARRAY = 12 << 20   # five arrays: at most 60 MiB per dump
+
+
+def dump_outputs(outdir, arrays):
+    """Writes each tensor as float32 <outdir>/<name>.npy.  A tensor larger than DUMP_BYTES_PER_ARRAY is replaced by a
+    fixed sample of its rows (first dimension): the sorted indices np.random.default_rng(0).choice(rows, k,
+    replace=False) with k = DUMP_BYTES_PER_ARRAY // row bytes, the same rows in every run of the same shape."""
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        rows = t.shape[0]
+        k = max(1, DUMP_BYTES_PER_ARRAY // (t[0].numel() * 4))
+        if k < rows:
+            idx = np.sort(np.random.default_rng(0).choice(rows, k, replace=False))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(outdir, name + ".npy"), t.cpu().numpy())
+
+
 def parity_check_sharded(rank, world, dev, B, d, R, transport=None):
     """N > 1: a small graph through the SAME sharded code path (device plan, overlapped halo exchange, gradient
     all-reduce) against the single-GPU layer computed on rank 0.  The driver's GPU test box has one GPU, so this is
@@ -352,7 +374,15 @@ def main():
     ap.add_argument("--triples-npz", default=None,
                     help="use the triples of this .npz (arrays: triples [E,3], V, R) instead of the synthetic generator; "
                          "diagnostic only (e.g. the real FB15k-237 graph), the default bench stays synthetic")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's out, dH and weight gradients to "
+                         "DIR/<name>.npy (float32; a fixed row sample of any array over 12 MiB); with N > 1 each rank "
+                         "writes its own under DIR/rank<r>/")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -458,10 +488,14 @@ def main():
         l0 = _lib.launch_count()
         sync_all()
         w0 = time.time()
+        last_out = None
         for i in range(args.steps):
             flush_buf.zero_()  # L2 flush between timed iterations (outside the event pair)
             ev0[i].record()
-            step()
+            if i + 1 < args.steps:
+                step()
+            else:
+                last_out = step()   # kept for --dump-outputs; earlier outputs are freed as they come
             ev1[i].record()
         sync_all()
         w1 = time.time()
@@ -470,9 +504,9 @@ def main():
             t = torch.tensor([ms], device=dev, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, w0, w1, _lib.launch_count() - l0
+        return ms, w0, w1, _lib.launch_count() - l0, last_out
 
-    total_ms, wall0, wall1, launches = timed_region()
+    total_ms, wall0, wall1, launches, last_out = timed_region()
     clocks = sampler.stop(wall0, wall1) if sampler else None
     remeasured = False
     bad = {"hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown"}
@@ -482,13 +516,19 @@ def main():
     if int(flag.item()):  # a throttled run is rejected and re-measured once (B200_PROFILING.md)
         sampler = ClockSampler(local_rank) if rank == 0 else None
         time.sleep(0.5)
-        total_ms, wall0, wall1, launches = timed_region()
+        last_out = None
+        total_ms, wall0, wall1, launches, last_out = timed_region()
         clocks = sampler.stop(wall0, wall1) if sampler else None
         remeasured = True
     if clocks is not None:
         clocks["remeasured_after_throttle"] = remeasured
     ms_per_step = total_ms / args.steps
     value = E / (ms_per_step * 1e-3) / 1e6
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, "rank%d" % rank),
+                     {"out": last_out, "dH": H.grad, "dW_forward": Wf.grad, "dW_backward": Wb.grad,
+                      "dW_self": Ws.grad})
+    last_out = None   # at full scale the output is 20 GB: released before the profiling and e2e legs
 
     # ---- per-stage timing (separate pass, events inside the library): roofline of the dominant kernel and of the layer
     peak, peak_src = peaks()

@@ -1,6 +1,7 @@
 """Golden vectors produced by RUNNING THE REFERENCE'S OWN MODEL CODE (needs /root/reference; run HERE):
 
   python tests/golden/make_reference_golden.py        ->  tests/golden/reference_model_golden.npz
+                                                          tests/golden/reference_model_golden_tf_kernel.npz
 
 The reference's model_builder / Representation / AffineTransform / ConcatGcn / BasisGcn / RelationEmbedding /
 BilinearDiag classes are imported unmodified from /root/reference/code and executed over tests/golden/tf1_shim.py
@@ -200,8 +201,21 @@ def main():
              [('Encoder', 'InternalEncoderDimension', '20'), ('Shared', 'CodeDimension', '12'),
               ('Encoder', 'NumberOfBasisFunctions', '4'), ('Encoder', 'UseOutputTransform', 'Yes')],
              toy_train, toy_test, tV, tR, 8, "canonical", out)
-    np.savez_compressed(os.path.join(HERE, "reference_model_golden.npz"), **out)
-    print("wrote reference_model_golden.npz (%d arrays)" % len(out))
+    # a tf_kernel case shares its inputs and weights with the canonical case of the same model: its own file holds
+    # only the arrays that differ, which keeps both fixtures under 1 MB (tests/test_reference_golden.py:load_case)
+    canonical, tf_kernel = {}, {}
+    for k, v in out.items():
+        case, arr = k.split("/")
+        if not case.endswith("_tf_kernel"):
+            canonical[k] = v
+            continue
+        twin = out[case[:-len("tf_kernel")] + "canonical/" + arr]
+        if not (v.dtype == twin.dtype and v.shape == twin.shape and v.tobytes() == twin.tobytes()):
+            tf_kernel[k] = v
+    np.savez_compressed(os.path.join(HERE, "reference_model_golden.npz"), **canonical)
+    np.savez_compressed(os.path.join(HERE, "reference_model_golden_tf_kernel.npz"), **tf_kernel)
+    print("wrote reference_model_golden.npz (%d arrays), reference_model_golden_tf_kernel.npz (%d arrays)"
+          % (len(canonical), len(tf_kernel)))
 
 
 if __name__ == "__main__":

@@ -1,6 +1,6 @@
-"""CPU, only where the reference checkout is mounted (/root/reference; skipped on the GPU box): the real
-datasets through OUR loaders + host graph preparation against the dataset-level integer goldens recorded by
-tests/golden/make_golden.py (SURVEY.md 8c)."""
+"""CPU: a fixed sample of the real datasets (tests/golden/real_datasets_sample.npz, made by
+tests/golden/make_dataset_samples.py) through OUR loaders + host graph preparation, against what the original
+project's loader made of the same text (SURVEY.md 8c)."""
 import os
 
 import numpy as np
@@ -10,21 +10,21 @@ from relationprediction_b200.common import io
 from relationprediction_b200.ops import Graph
 from relationprediction_b200 import _lib
 
-REF = "/root/reference/data"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference datasets not mounted")
+SAMPLE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "real_datasets_sample.npz")
 
 
 @pytest.mark.parametrize("name", ["FB-Toutanova", "wn18", "FB15k"])
-def test_dataset_goldens_and_graph_invariants(toy, name):
+def test_dataset_goldens_and_graph_invariants(toy, tmp_path, name):
     gold = toy["dataset_stats"][name]
-    d = os.path.join(REF, name)
-    tr = io.read_triplets_as_array(os.path.join(d, "train.txt"), os.path.join(d, "entities.dict"),
-                                   os.path.join(d, "relations.dict"))
+    z = np.load(SAMPLE)
+    for fname in ("train.txt", "entities.dict", "relations.dict"):
+        (tmp_path / fname).write_bytes(z["%s/%s" % (name, fname)].tobytes())
+    tr = io.read_triplets_as_array(str(tmp_path / "train.txt"), str(tmp_path / "entities.dict"),
+                                   str(tmp_path / "relations.dict"))
     V, R = gold["V"], gold["R"]
-    assert tr.shape == (gold["E_train"], 3) and tr[:5].tolist() == gold["first_triples"]
-    assert [int(tr[:, k].astype(np.int64).sum()) for k in range(3)] == gold["checksum_s_r_o"]
-    deg = np.bincount(np.concatenate([tr[:, 0], tr[:, 2]]), minlength=V)
-    assert int((deg == 0).sum()) == gold["isolated"] and int(deg.max()) == gold["max_degree"]
+    assert (int(z[name + "/V"]), int(z[name + "/R"])) == (V, R)
+    np.testing.assert_array_equal(tr, z[name + "/triples"])
+    assert tr.dtype == np.int32 and len(tr) > 1000
     g = Graph(tr, V, R)   # host-side build
     info = g.info()
     assert info[0] == 2 * len(tr) and info[3] == 2 * R
@@ -39,8 +39,6 @@ def test_dataset_goldens_and_graph_invariants(toy, name):
         sel = (relw >= lo) & (relw < hi)
         sums = np.bincount(rows[sel], weights=norm[sel].astype(np.float64), minlength=V)
         assert np.all((np.abs(sums - 1) < 1e-4) | (sums == 0))
-    # (dst, weight id) run count reported by the library == independent count
+    # (dst, weight id) run count reported by the library == independent count == the count recorded with the sample
     key = rows.astype(np.int64) * (2 * R) + relw
-    assert info[9] == 1 + int((key[1:] != key[:-1]).sum())
-    if name == "FB-Toutanova":
-        assert info[9] == 149689   # 544 230 messages collapse to 149 689 block mat-vecs (DESIGN.md)
+    assert info[9] == 1 + int((key[1:] != key[:-1]).sum()) == int(z[name + "/runs"])

@@ -15,6 +15,7 @@ import torch
 from oracle import rgcn_oracle as oracle
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_model_golden.npz")
+GOLDEN_TF_KERNEL = os.path.join(os.path.dirname(GOLDEN), "reference_model_golden_tf_kernel.npz")
 CASES = [(n, v) for n, v in [("block_toy_s5", "block"), ("block_syn_s8", "block"), ("basis_toy", "basis"),
                              ("basis_syn", "basis")]]
 GROUPINGS = [("tf_kernel", "tf_unsorted_compat"), ("canonical", "canonical")]
@@ -22,10 +23,20 @@ KEEP = 0.8           # DropoutKeepProbability of both shipped settings files
 LAMBDA = 0.01        # RegularizationParameter of both shipped settings files
 
 
-def load_case(name):
-    z = np.load(GOLDEN)
+def _case_arrays(path, name):
+    z = np.load(path)
     p = name + "/"
     return {k[len(p):]: z[k] for k in z.files if k.startswith(p)}
+
+
+def load_case(name):
+    """A tf_kernel case is stored as the arrays in which it differs from the canonical case of the same model
+    (inputs and weights are shared); tests/golden/make_reference_golden.py writes both files."""
+    if name.endswith("_tf_kernel"):
+        c = _case_arrays(GOLDEN, name[:-len("tf_kernel")] + "canonical")
+        c.update(_case_arrays(GOLDEN_TF_KERNEL, name))
+        return c
+    return _case_arrays(GOLDEN, name)
 
 
 # settings file + the overrides the generator applied, per golden case (shared by the CPU-chain and GPU tests)
