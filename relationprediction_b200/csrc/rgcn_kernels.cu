@@ -1177,11 +1177,20 @@ bool block_rel_supported(int d, int s) {
   return false;
 }
 
+// s = 5: warps per group of the group kernel k_block_relg (4 by default; $RGCN_REL_GROUP = 2 | 4, any other value
+// selects the one-warp kernel k_block_rel<5, NV, false>)
+static int rel_group_s5() {
+  int G = 4;
+  if (const char* e = std::getenv("RGCN_REL_GROUP")) G = std::atoi(e);
+  return G;
+}
+
 // the dW-fused variant keeps 2*s*NV float4 of weights + gradient accumulators in registers
 bool block_rel_fuse_dw_supported(int d, int s) {
   if (s == 5) {  // group-kernel variant: dH+dW in one walk measured 0.62 ms vs 0.34 + 0.38 ms separate
     const char* e = std::getenv("RGCN_FUSE_DW_S5");
-    return d <= 512 && !(e && std::atoi(e) == 0);
+    const int G = rel_group_s5();
+    return d <= 512 && !(e && std::atoi(e) == 0) && (G == 4 || G == 2);  // only the group kernel fuses dW
   }
   return s == 4 || s == 8 || s == 16;
 }
@@ -1191,28 +1200,24 @@ int launch_block_rel(const WorkItem* items, int n_items, const int32_t* r_row, c
                      float* out, const float* Hrow, int ldh, float* dWt, cudaStream_t st) {
   if (n_items == 0) return RGCN_OK;
   const bool fuse = dWt != nullptr;
-  if (fuse && !block_rel_fuse_dw_supported(d, s) && s != 5) {
-    rgcn_set_error("rel-major block kernel: dW fusion unsupported for this block size");
+  if (fuse && !block_rel_fuse_dw_supported(d, s)) {
+    rgcn_set_error("rel-major block kernel: dW fusion unsupported for this block size / kernel choice");
     return RGCN_ERR_INVALID;
   }
-#define RL(S_, NV_)                                                                                  \
-  return fuse ? launch_block_rel_t<S_, NV_, true>(items, n_items, r_row, r_nbr, r_norm, X, ldx, d, Wt, \
-                                                  out, Hrow, ldh, dWt, st)                             \
-              : launch_block_rel_t<S_, NV_, false>(items, n_items, r_row, r_nbr, r_norm, X, ldx, d,   \
-                                                   Wt, out, Hrow, ldh, dWt, st)
+  // the dW-fused variant doubles the per-lane register state: it runs with ONE quad per lane (4 column slabs at
+  // d = 512; keeps two blocks per SM resident and measured fastest, 11.4 vs 12.6 ms/step, synthetic), the only
+  // fused instantiation
+#define RLF(S_) \
+  return launch_block_rel_t<S_, 1, true>(items, n_items, r_row, r_nbr, r_norm, X, ldx, d, Wt, out, Hrow, ldh, dWt, st)
 #define RLN(S_, NV_) \
   return launch_block_rel_t<S_, NV_, false>(items, n_items, r_row, r_nbr, r_norm, X, ldx, d, Wt, out, Hrow, ldh, dWt, st)
   int nv = pick_nv(d);
-  // the dW-fused variant doubles the per-lane register state: one quad per lane (4 column slabs at
-  // d = 512) keeps two blocks per SM resident and measured fastest (11.4 vs 12.6 ms/step, synthetic)
-  if (fuse && s != 5) nv = 1;
   if (const char* e = std::getenv("RGCN_REL_NV")) {  // tuning knob: quads per lane (column slabs = d/(128 nv))
     const int v = std::atoi(e);
     if (v >= 1 && v <= 4 && s != 5 && (v * 128) % s == 0) nv = std::min(nv, v);
   }
   if (s == 5) {
-    int G = 4;
-    if (const char* e = std::getenv("RGCN_REL_GROUP")) G = std::atoi(e);
+    const int G = rel_group_s5();
     if (G == 4 || G == 2) {
       const int groups = RGCN_WARPS_PER_BLOCK / G;
       dim3 grid((n_items + groups - 1) / groups);
@@ -1230,15 +1235,19 @@ int launch_block_rel(const WorkItem* items, int n_items, const int32_t* r_row, c
       return check_launch("k_block_relg");
     }
     switch (nv) { case 1: RLN(5, 1); case 2: RLN(5, 2); case 3: RLN(5, 3); default: RLN(5, 4); }
+  } else if (fuse) {
+    if (s == 4) RLF(4);
+    if (s == 8) RLF(8);
+    RLF(16);
   } else if (s == 4) {
-    switch (nv) { case 1: RL(4, 1); case 2: RL(4, 2); case 3: RL(4, 3); default: RL(4, 4); }
+    switch (nv) { case 1: RLN(4, 1); case 2: RLN(4, 2); case 3: RLN(4, 3); default: RLN(4, 4); }
   } else if (s == 8) {
-    if (nv == 1) RL(8, 1);
-    RL(8, 2);
+    if (nv == 1) RLN(8, 1);
+    RLN(8, 2);
   } else if (s == 16) {
-    RL(16, 1);
+    RLN(16, 1);
   }
-#undef RL
+#undef RLF
 #undef RLN
   rgcn_set_error("rel-major block kernel: unsupported block size");
   return RGCN_ERR_INVALID;
